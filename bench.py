@@ -120,7 +120,7 @@ class ClockSampler:
 
 # ------------------------------------------------------------------ CPU arms
 
-def cpu_pipeline(steps: int, warmup: int, size: int = 0):
+def cpu_pipeline(steps: int, warmup: int, size: int = 0, dump_dir=None):
     """The reference's CPU implementation (oracle/_ref when present, else the oracle port): blur sigma=4 then Lanczos 2x
     down on one size^2 RGBA image per step, all host threads.  size defaults to the GPU arm's 8192 (the CPU test suite
     shrinks it through MB200_BENCH_CPU_SIZE to stay fast on small machines; the `sample` string always says what ran)."""
@@ -160,6 +160,8 @@ def cpu_pipeline(steps: int, warmup: int, size: int = 0):
     for _ in range(steps):
         step()
     dt = time.perf_counter() - t0
+    if dump_dir:
+        dump_outputs(dump_dir, out)
     name = "ImageMagick 7.1.1-45 Q16-HDRI OpenMP" if kind == "reference" else "oracle port"
     return {"value": steps * n * n / dt / 1e6, "unit": "Mpixels/s", "cores": cores, "kind": kind,
             "sample": f"{steps} x ({n}x{n} RGBA BlurImage(0,{SIGMA}) + ResizeImage {n // 2}x{n // 2} Lanczos), {name}, "
@@ -169,7 +171,7 @@ def cpu_pipeline(steps: int, warmup: int, size: int = 0):
 def run_reference(args):
     if int(os.environ.get("RANK", "0")) != 0:
         return 0
-    cpu, ms = cpu_pipeline(max(1, args.steps), max(1, min(args.warmup, 2)))
+    cpu, ms = cpu_pipeline(max(1, args.steps), max(1, min(args.warmup, 2)), dump_dir=args.dump_outputs)
     line = {"impl": "reference", "metric": METRIC, "value": cpu["value"], "unit": "Mpixels/s",
             "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
@@ -216,6 +218,22 @@ def gpu_cpu_affinity(index: int):
     except Exception:
         pass
     return None, None
+
+
+DUMP_ROWS = 512           # rows of a 4096 x 4096 RGBA result kept by --dump-outputs (32 MB)
+
+
+def dump_outputs(directory, pixels):
+    """What the last timed step returned -- the Lanczos result of the step's last image, an (H, W, 4) numpy array or
+    tensor -- as DIR/lanczos_rows.npy in float32: a seeded, fixed choice of min(H, DUMP_ROWS) of its rows (the same rows
+    in every run), so two builds can be compared output for output.  Written by rank 0 only."""
+    rows = np.sort(np.random.default_rng(0).choice(pixels.shape[0], min(pixels.shape[0], DUMP_ROWS), replace=False))
+    sample = pixels[rows.tolist()]
+    if not isinstance(sample, np.ndarray):
+        sample = sample.float().cpu().numpy()
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "lanczos_rows.npy", np.ascontiguousarray(sample, np.float32))
 
 
 def run_gpu(args):
@@ -331,7 +349,7 @@ def run_gpu(args):
     t_start, t_end = ev(), ev()
     t_start.record()
     for _ in range(args.steps):
-        run_step()
+        step_out = run_step()
     t_end.record()
     torch.cuda.synchronize()
     clk_t1 = time.perf_counter()
@@ -345,6 +363,8 @@ def run_gpu(args):
     clock_summary = clocks.summary(clk_t0, clk_t1) if clocks else None
     if clocks:
         clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, (graph_out if graph is not None else step_out).pixels)
 
     # ---- roofline inputs: each pass of the blur alone (events around exactly one launch), FP64 issue-rate probe
     row_k, col_k = im.AcquireKernelInfo(f"blur:0x{SIGMA}"), im.AcquireKernelInfo(f"blur:0x{SIGMA}+90")
@@ -515,7 +535,7 @@ def run_gpu(args):
     pageable_ms = e2e_run(4, False, 1) if world == 1 else None
     if rank == 0:
         e2e_modes["eager_pageable_ms_per_image"] = pageable_ms
-        harness = ROOT / "imagemagick_b200" / "lib" / "chain_harness"
+        harness = ROOT / "oracle" / "_ref" / "shim" / "chain_harness"
         if world == 1 and harness.exists():                   # BlurImage -> ResizeImage through the MagickCore shim itself
             try:
                 r = subprocess.run([str(harness), str(SIZE), "3", "0"], capture_output=True, text=True, timeout=600)
@@ -644,7 +664,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--streams", type=int, default=int(os.environ.get("BENCH_STREAMS", "1")),
                     help="image-parallel branches of the timed step's CUDA graph (independent images on separate streams)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of what the last step computed to DIR/*.npy "
+                         "(rank 0; with --impl reference, the reference's result)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)

@@ -199,23 +199,21 @@ def test_bench_reference_arm_contract():
     assert "1024x1024" in line["cpu_baseline"]["sample"]          # this test shrinks the sample; the driver runs 8192^2
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref not built")
 def test_sharpen_and_edge_kernels_match_the_reference_taps():
     """effect.c:3991 / :1520 build their kernels inline; convolving a one-pixel impulse with the real
     SharpenImage / EdgeImage returns those taps (reflected), which must equal the product's host-built kernels."""
     lib = _lib.load()
     for name, build, ref_call in (
-            ("sharpen", lambda: lib.mb200_sharpen_kernel(0.0, 1.0), lambda s, d, n: util.ref().ref_sharpen(util.P(s), util.P(d), n, n, 1, 0.0, 1.0)),
-            ("sharpen r2", lambda: lib.mb200_sharpen_kernel(2.0, 0.7), lambda s, d, n: util.ref().ref_sharpen(util.P(s), util.P(d), n, n, 1, 2.0, 0.7)),
-            ("edge", lambda: lib.mb200_edge_kernel(1.0), lambda s, d, n: util.ref().ref_edge(util.P(s), util.P(d), n, n, 1, 1.0))):
+            ("sharpen", lambda: lib.mb200_sharpen_kernel(0.0, 1.0), lambda s, n: util.ref_output("ref_sharpen", s, util.OUT, n, n, 1, 0.0, 1.0, shape=s.shape)),
+            ("sharpen r2", lambda: lib.mb200_sharpen_kernel(2.0, 0.7), lambda s, n: util.ref_output("ref_sharpen", s, util.OUT, n, n, 1, 2.0, 0.7, shape=s.shape)),
+            ("edge", lambda: lib.mb200_edge_kernel(1.0), lambda s, n: util.ref_output("ref_edge", s, util.OUT, n, n, 1, 1.0, shape=s.shape))):
         k = im.KernelInfo(build())
         vals, kx, ky = k.arrays()[0]
         w = vals.shape[0]
         n = w + 8
         src = np.zeros((n, n, 1), np.float32)
         src[n // 2, n // 2, 0] = 1.0
-        dst = np.empty_like(src)
-        assert ref_call(src, dst, n) == 0
+        dst = ref_call(src, n)
         got = dst[n // 2 - ky: n // 2 - ky + w, n // 2 - kx: n // 2 - kx + w, 0]
         want = vals[::-1, ::-1].astype(np.float32)          # convolution reflects the kernel
         assert np.array_equal(got, want), name
@@ -260,9 +258,9 @@ def test_process_filter_module_on_the_cpu_path():
     must reproduce the stock operators bit for bit, keep the list intact and reject unknown operators."""
     import os
     import subprocess
-    exe = ROOT / "imagemagick_b200" / "lib" / "filter_harness"
+    exe = util.SHIM_DIR / "filter_harness"
     if not exe.exists():
-        pytest.skip("filter_harness not built (needs the reference tree: python __graft_entry__.py)")
+        pytest.skip("filter_harness not built (needs an ImageMagick source tree: IMAGEMAGICK_SOURCE=<tree> python __graft_entry__.py)")
     env = dict(os.environ)
     if _lib.load().mb200_device_count() == 0:
         env["B200_FILTER_EXPECT_EXACT"] = "1"
@@ -276,9 +274,9 @@ def test_wrapped_entry_points_fall_back_on_the_cpu():
     declines silently and returns exactly what the stock function returns -- including __wrap_ThumbnailImage,
     whose cascade is re-issued by the shim and whose Thumb::* metadata comes from the real function."""
     import subprocess
-    exe = ROOT / "imagemagick_b200" / "lib" / "shim_harness"
+    exe = util.SHIM_DIR / "shim_harness"
     if not exe.exists():
-        pytest.skip("shim_harness not built (needs the reference tree: python __graft_entry__.py)")
+        pytest.skip("shim_harness not built (needs an ImageMagick source tree: IMAGEMAGICK_SOURCE=<tree> python __graft_entry__.py)")
     if _lib.load().mb200_device_count() != 0:
         pytest.skip("device present: the GPU variant of this check is tests/test_gpu_parity.py::test_magickcore_shim_end_to_end")
     p = subprocess.run([str(exe)], capture_output=True, text=True, timeout=600)
@@ -287,7 +285,6 @@ def test_wrapped_entry_points_fall_back_on_the_cpu():
     assert p.stdout.count("ThumbnailImage RGBA") == 3
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("rad,sig,ang", [(0, 2, 0), (0, 2, 45), (0, 3, 90), (0, 1.5, -30), (0, 4, 180), (5, 2, 270), (0, 2, 123.4)])
 def test_motion_blur_taps_and_offsets_match_the_reference(rad, sig, ang):
     """The product builds MotionBlurImage's taps / offsets on the host (effect.c:2316-2345, :2390-2398); the real
@@ -300,12 +297,10 @@ def test_motion_blur_taps_and_offsets_match_the_reference(rad, sig, ang):
     c = size // 2
     src = np.zeros((size, size, 1), np.float32)
     src[c, c, 0] = 1.0
-    dst = np.empty_like(src)
-    assert util.ref().ref_motion_blur(util.P(src), util.P(dst), size, size, 1, rad, sig, ang) == 0
     want = np.zeros((size, size), np.float64)
     for j in range(n):                      # out[y][x] = sum_j k_j * src[y + oy_j][x + ox_j], accumulated in tap order
         want[c - oy[j], c - ox[j]] += t[j]
-    assert np.array_equal(dst[..., 0], want.astype(np.float32))
+    util.expect_ref(want.astype(np.float32)[..., None], "ref_motion_blur", src, util.OUT, size, size, 1, rad, sig, ang)
 
 
 @pytest.mark.parametrize("sizes", [((37, 23), (19, 11)), ((20, 14), (53, 31)), ((31, 17), (31, 9)), ((64, 8), (21, 8))])

@@ -2,6 +2,8 @@
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
+import os
 from pathlib import Path
 
 import numpy as np
@@ -9,6 +11,7 @@ import numpy as np
 ROOT = Path(__file__).resolve().parent.parent
 ORACLE_SO = ROOT / "oracle" / "liboracle.so"
 REF_SO = ROOT / "oracle" / "_ref" / "libmagickref.so"
+SHIM_DIR = ROOT / "oracle" / "_ref" / "shim"      # MagickCore shim harnesses (imagemagick_b200/shim/Makefile)
 
 _fp = C.POINTER(C.c_float)
 _sz, _d, _i, _l = C.c_size_t, C.c_double, C.c_int, C.c_long
@@ -89,10 +92,6 @@ def oracle() -> C.CDLL:
     return _oracle
 
 
-def have_ref() -> bool:
-    return REF_SO.exists()
-
-
 def ref() -> C.CDLL:
     """The real reference (ImageMagick compiled from source); only exists where
     oracle/_ref has been built (this container / shipped prebuilt to the GPU box)."""
@@ -138,6 +137,147 @@ def ref_kernel(string: str, idx: int = 0):
     if rc:
         return None
     return np.array(vals[: kw.value * kh.value]).reshape(kh.value, kw.value), kx.value, ky.value
+
+
+# ---- the reference's outputs, stored ----------------------------------------------------------------------------------
+# Tests that compare with the reference read what it computed from REF_GOLDEN, so they run without the reference tree.
+# A call is identified by the function name, its arguments (input pixels by content) and how it is compared; what is
+# stored is a 64-bit digest of the return code and of the output with every float32 mapped to its sign-magnitude
+# integer (the relation max_ulp(a, b) == 0 is equality of those integers) or, for exact_bits, to its bit pattern; for
+# ref_output() and stored_ref_kernel(), the arrays themselves.
+# MB200_RECORD_REF_OUTPUTS=1 runs the real library (oracle/_ref) instead and checks against it;
+# tests/golden/make_ref_outputs.py then writes what it returned (save_recording()).
+REF_GOLDEN = ROOT / "tests" / "golden" / "ref_outputs.npz"
+RECORD = os.environ.get("MB200_RECORD_REF_OUTPUTS") == "1"
+REGENERATE = ("tests/golden/make_ref_outputs.py (needs oracle/_ref/libmagickref.so; it also runs this comparison against "
+              "the live library, element by element)")
+OUT = object()              # argument placeholder: the output buffer
+
+
+class InOut:
+    """Argument placeholder: an output buffer that starts as a copy of `a` (operators that work in place)."""
+
+    def __init__(self, a: np.ndarray):
+        self.a = a
+
+
+_store = None
+
+
+def save_recording():
+    """Writes what the recording run returned to REF_GOLDEN.  Digests go into two uint64 columns (call, output), sorted
+    by call; arrays are stored under their own names."""
+    assert RECORD and _store
+    digests = sorted((int(k[2:], 16), int(v, 16)) for k, v in _store.items() if k.startswith("d:"))
+    arrays = {k: v for k, v in _store.items() if not k.startswith("d:")}
+    np.savez_compressed(REF_GOLDEN, digests=np.array(digests, np.uint64).reshape(-1, 2), **arrays)
+
+
+def _golden():
+    global _store
+    if _store is None:
+        if RECORD:
+            _store = {}
+        else:
+            with np.load(REF_GOLDEN) as z:
+                _store = {k: z[k] for k in z.files if k != "digests"}
+                _store.update((f"d:{int(k):016x}", f"{int(v):016x}") for k, v in z["digests"])
+    return _store
+
+
+def _hash(*parts) -> str:
+    h = hashlib.blake2b(digest_size=8)
+    for p in parts:
+        if isinstance(p, InOut):
+            p = ("inout", p.a)
+        if isinstance(p, tuple):
+            h.update(_hash(*p).encode())
+        elif isinstance(p, np.ndarray):
+            h.update(repr((p.dtype.str, p.shape)).encode())
+            h.update(np.ascontiguousarray(p).tobytes())
+        else:
+            if isinstance(p, (np.integer, np.floating)):
+                p = p.item()
+            h.update(repr("out" if p is OUT else p).encode())
+    return h.hexdigest()
+
+
+def _live_call(fn, args, out_shape):
+    out = None
+    call = []
+    for a in args:
+        if a is OUT:
+            out = np.empty(out_shape, np.float32)
+            a = out
+        elif isinstance(a, InOut):
+            out = a = a.a.copy()
+        call.append(P(a) if isinstance(a, np.ndarray) else a)
+    return getattr(ref(), fn)(*call), out
+
+
+def _comparable(a: np.ndarray, mode: str) -> np.ndarray:
+    """The integers whose equality is the comparison: "bits" the float32 bit patterns; "ulp" the sign-magnitude order
+    (max_ulp == 0); "nan" the same with every NaN mapped to one value."""
+    i = np.ascontiguousarray(a, np.float32).view(np.int32).astype(np.int64)
+    if mode == "bits":
+        return i
+    k = np.where(i < 0, -(i & 0x7FFFFFFF), i)
+    return np.where(np.isnan(a), np.int64(1) << 40, k) if mode == "nan" else k
+
+
+def expect_ref(got, fn: str, *args, rc: int = 0, nan_equal: bool = False, exact_bits: bool = False,
+               threads: int = 0) -> None:
+    """Asserts that the reference's `fn(*args)` returned `rc` and wrote `got`: max_ulp == 0; with nan_equal, NaN wherever
+    the reference has NaN, in any encoding; with exact_bits, the same float32 bit patterns.  `got` None: only the
+    return code is compared.  `threads`: the reference's thread count for the call."""
+    mode = "rc" if got is None else "bits" if exact_bits else "nan" if nan_equal else "ulp"
+    key = "d:" + _hash(fn, threads, mode, *args)
+    if RECORD:
+        if threads:
+            ref().ref_set_threads(threads)
+        want_rc, want = _live_call(fn, args, None if got is None else got.shape)
+        _golden()[key] = _output_digest(want_rc, want, mode)
+        assert want_rc == rc, (fn, want_rc)
+        if got is not None:
+            d = _comparable(got, mode) != _comparable(want, mode)
+            assert not d.any(), (fn, f"{int(d.sum())} elements differ, first at {np.argwhere(d)[0].tolist()}",
+                                 f"max ULP {max_ulp(got, want)}")
+        return
+    stored = _golden().get(key)
+    assert stored is not None, f"{fn}: no stored reference output for this call; regenerate with {REGENERATE}"
+    assert stored == _output_digest(rc, got, mode), \
+        f"{fn}: differs from the reference's output; where and by how much: {REGENERATE}"
+
+
+def _output_digest(rc: int, out, mode: str) -> str:
+    return _hash(rc, None if mode == "rc" else _comparable(out, mode))
+
+
+def ref_output(fn: str, *args, shape) -> np.ndarray:
+    """The array the reference's `fn(*args)` wrote into its OUT argument of the given shape (asserting it returned 0)."""
+    key = "a:" + _hash(fn, shape, *args)
+    if RECORD:
+        rc, out = _live_call(fn, args, shape)
+        assert rc == 0, (fn, rc)
+        _golden()[key] = out
+    out = _golden().get(key)
+    assert out is not None, f"{fn}: no stored reference output for this call; regenerate with {REGENERATE}"
+    return out
+
+
+def stored_ref_kernel(string: str, idx: int = 0):
+    """ref_kernel() as stored: the reference's kernel list element `idx` for a kernel string as (values, x, y), None
+    past the end of the list."""
+    key = "k:" + _hash(string, idx)
+    if RECORD:
+        k = ref_kernel(string, idx)
+        _golden()[key] = np.zeros(0) if k is None else np.concatenate([[k[1], k[2], k[0].shape[1]], k[0].ravel()])
+    flat = _golden().get(key)
+    assert flat is not None, f"{string}: no stored reference kernel; regenerate with {REGENERATE}"
+    if flat.size == 0:
+        return None
+    x, y, w = (int(v) for v in flat[:3])
+    return flat[3:].reshape(-1, w), x, y
 
 
 def orc_kernel(kind: str, rho=0.0, sigma=0.0, xi=0.0, psi=0.0) -> OrcKernel:
